@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W                      # this repo's CUDA engine
     python bench.py --impl reference --gpus N --steps K --warmup W     # the reference's own CPU path
     python bench.py --config cfg3|cfg4|cfg5 ...                        # BASELINE.json configs[2..4] as their own lines
+    python bench.py ... --dump-outputs DIR                             # also write the last timed step's outputs (.npy)
 
 Default workload ("pairs"): one step per GPU = one pass of the hot path over 1024 synthetic image-text pairs:
 vision tower (224x224, bf16 pixels resident in HBM) + text tower (77-token ids) + L2-normalise + logits_per_image
@@ -437,13 +438,16 @@ class Timer:
             dist.barrier()
         torch.cuda.synchronize()
 
-    def timed(self, fn, steps):
-        """barrier + sync, CUDA events on the launch stream around `steps` calls, barrier + sync, MAX over ranks (ms)."""
+    def timed(self, fn, steps, keep_last=False):
+        """barrier + sync, CUDA events on the launch stream around `steps` calls, barrier + sync, MAX over ranks (ms).
+        With `keep_last`, returns (ms, what the last call returned)."""
         self.barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        out = None
         e0.record()
         for i in range(steps):
-            fn(i)
+            out = None          # release the previous step's result before the next step runs, as if it were discarded
+            out = fn(i)
         e1.record()
         self.barrier()
         ms = e0.elapsed_time(e1)
@@ -452,7 +456,39 @@ class Timer:
             t = torch.tensor([ms], device=self.dev)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = float(t.item())
-        return ms
+        return (ms, out) if keep_last else ms
+
+
+DUMP_BYTES = 64 << 20          # --dump-outputs writes at most this much per run
+DUMP_ARRAY_BYTES = 16 << 20    # a larger array is written as a seeded sample of its rows
+
+
+def dump_outputs(ctx, arrays):
+    """--dump-outputs DIR (rank 0): the arrays the timed path returned in its last step, as DIR/<name>.npy, so that two
+    builds can be compared output for output.  Floating-point arrays are written as float32, integer ones as float64
+    (exact).  An array above DUMP_ARRAY_BYTES keeps a sorted sample of its rows, drawn with a fixed seed from the row
+    count alone (the same rows in every run); the row numbers go to DIR/<name>_rows.npy."""
+    path = ctx["args"].dump_outputs
+    if not path or ctx["rank"] != 0:
+        return
+    os.makedirs(path, exist_ok=True)
+    total = 0
+    for name, t in arrays.items():
+        t = t.detach()
+        dtype = torch.float32 if t.is_floating_point() else torch.float64
+        elem = 4 if dtype == torch.float32 else 8
+        if t.numel() * elem > DUMP_ARRAY_BYTES:
+            n = t.shape[0]
+            k = max(1, DUMP_ARRAY_BYTES // (t[0].numel() * elem))
+            rows = np.sort(np.random.default_rng(0).choice(n, size=k, replace=False))
+            np.save(os.path.join(path, f"{name}_rows.npy"), rows.astype(np.float64))
+            total += rows.size * 8
+            t = t.index_select(0, torch.from_numpy(rows).to(t.device))
+        a = t.to(dtype).cpu().numpy()
+        np.save(os.path.join(path, f"{name}.npy"), a)
+        total += a.nbytes
+    if total > DUMP_BYTES:
+        raise RuntimeError(f"--dump-outputs wrote {total} bytes, more than {DUMP_BYTES}")
 
 
 def run_ours(args):
@@ -533,10 +569,12 @@ def bench_pairs(ctx):
     timer.barrier()
     launches0 = L.plip_launch_count()
     t_wall0 = time.time()
-    ms = timer.timed(step, args.steps)
+    ms, lpi = timer.timed(step, args.steps, keep_last=True)
     t_wall1 = time.time()
     launches = L.plip_launch_count() - launches0
     clocks = sampler.stop(t_wall0, t_wall1) if sampler else None
+    dump_outputs(ctx, {"logits_per_image": lpi})
+    del lpi
     ms_per_step = ms / args.steps
     value = PAIRS * ws * args.steps / (ms / 1e3)
 
@@ -706,17 +744,20 @@ def bench_cfg3(ctx):
     ids = ids.to(dev)
 
     def step(i):
-        return model(input_ids=ids, pixel_values=px).logits_per_image
+        return model(input_ids=ids, pixel_values=px)
 
     sampler = ClockSampler(dev.index) if rank == 0 else None
     for i in range(args.warmup):
         step(i)
     launches0 = L.plip_launch_count()
     t0 = time.time()
-    ms = timer.timed(step, args.steps)
+    ms, out = timer.timed(step, args.steps, keep_last=True)
     t1 = time.time()
     launches = L.plip_launch_count() - launches0
     clocks = sampler.stop(t0, t1) if sampler else None
+    # logits_per_text is the transpose of logits_per_image
+    dump_outputs(ctx, {k: out[k] for k in ("logits_per_image", "image_embeds", "text_embeds")})
+    del out
     tiles_h = torch.from_numpy(synth.tiles_u8(n_img, seed=100)).pin_memory()
     ids_h = synth.token_ids(n_txt, seed=200, full_length=True)[0].pin_memory()
     out_h = torch.empty(n_img, n_txt, dtype=torch.float32).pin_memory()
@@ -773,10 +814,12 @@ def bench_cfg4(ctx):
         step(i)
     launches0 = L.plip_launch_count()
     t0 = time.time()
-    ms = timer.timed(step, args.steps)
+    ms, (pred, logits, all_img) = timer.timed(step, args.steps, keep_last=True)
     t1 = time.time()
     launches = L.plip_launch_count() - launches0
     clocks = sampler.stop(t0, t1) if sampler else None
+    dump_outputs(ctx, {"pred": pred, "logits": logits, "image_embeds": all_img})
+    del pred, logits, all_img
     # e2e: the same flow fed from a pinned host ring of 2 x 1024 tiles, H2D of every micro-batch inside the timed region
     ring = [torch.from_numpy(synth.tiles_u8(PAIRS, seed=100 + rank + i)).pin_memory() for i in range(2)]
     pred_h = torch.empty(n_local, dtype=torch.int64).pin_memory()
@@ -839,12 +882,14 @@ def bench_cfg5(ctx):
         step(i)
     launches0 = L.plip_launch_count()
     t0 = time.time()
-    ms = timer.timed(step, args.steps)
+    ms, block = timer.timed(step, args.steps, keep_last=True)
     t1 = time.time()
     launches = L.plip_launch_count() - launches0
     clocks = sampler.stop(t0, t1) if sampler else None
-    # the similarity block and the fused top-k head alone
     gal, q_all = state["gal"], state["q_all"]
+    dump_outputs(ctx, {"similarity": block, "gallery_embeds": gal, "query_embeds": q_all})
+    del block
+    # the similarity block and the fused top-k head alone
     sh.similarity(gal, q_all, sh.logit_scale_exp)
     sh.retrieval_topk(gal, q_all, 50, n_gal)                      # untimed first calls: scratch growth, lazy module loading
     ms_sim = timer.timed(lambda i: sh.similarity(gal, q_all, sh.logit_scale_exp), 3) / 3
@@ -902,10 +947,17 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-context", action="store_true", help="skip the stock-PyTorch-on-GPU context measurement")
     ap.add_argument("--quick", action="store_true", help="skip the extras (kernels alone, product-API extras, context)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed path returned in its last step (rank 0) as DIR/<name>.npy, at most 64 MB; "
+                         "one config, --impl ours")
     args = ap.parse_args()
     for c in args.config.split(","):
         if c not in WORKLOADS:
             ap.error(f"unknown config {c!r}")
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or "," in args.config):
+        ap.error("--dump-outputs needs --impl ours and a single config")
     if args.impl == "reference":
         args.config = args.config.split(",")[0]
         if args.steps is None:

@@ -13,7 +13,7 @@ What is pinned (the reference has no tests / fixtures of its own, SURVEY.md §4)
     heads ``_cosine_similarity`` / ``_nearest_neighbours``;
   * ``CLIPImageProcessor`` on non-224 images (resize + centre-crop + normalise).
 Weights are regenerated from the seed at test time (bit-reproducible torch CPU generator), so only
-outputs are stored.
+outputs are stored, plus one of the processor's two input images (the other is regenerated from its seed).
 """
 import os
 import sys
@@ -96,7 +96,7 @@ def main():
     rng = np.random.default_rng(9)
     big = [rng.integers(0, 256, (300, 260, 3), dtype=np.uint8), rng.integers(0, 256, (224, 512, 3), dtype=np.uint8)]
     pv = proc(images=[PIL.Image.fromarray(b) for b in big], return_tensors="pt")["pixel_values"].numpy()
-    out["proc_input_0"], out["proc_input_1"] = big[0], big[1]
+    out["proc_input_1"] = big[1]                    # big[0] is regenerated from the seed at test time (file < 1 MB)
     out["proc_pixel_values_sub"] = pv[:, :, ::8, ::8].copy()   # 28x28 subsample of the processor output
     out["proc_pixel_values_mean"] = pv.mean(axis=(2, 3))
     out["proc_class"] = np.array(type(proc).__name__)

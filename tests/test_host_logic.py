@@ -55,7 +55,8 @@ def test_preprocess_resize_crop_matches_clip_image_processor(golden):
     """Non-224 inputs: shortest-edge-224 bicubic + centre crop, then the device-side (x/255-mean)/std.
     Compared with the reference's CLIPImageProcessor output stored in the golden file."""
     from oracle import clip_oracle as O
-    imgs = [golden["proc_input_0"], golden["proc_input_1"]]
+    # the first input is regenerated from its seed (tests/golden/make_golden.py), the second is stored
+    imgs = [np.random.default_rng(9).integers(0, 256, (300, 260, 3), dtype=np.uint8), golden["proc_input_1"]]
     tiles = P.to_uint8_tiles(imgs)
     assert tiles.shape == (2, 224, 224, 3)
     pv = O.preprocess_u8(torch.from_numpy(tiles)).numpy()
